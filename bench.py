@@ -4,7 +4,7 @@
 A "step" is one full search of the workload's candidate space (every inter-stage plan enumerated by
 InterStagePlanGenerator, its intra-stage chain, load balancer and cost model) by libmetis_b200.so.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 Workload: BASELINE.json configs[2] ("homo 64-GPU cluster, 96-layer GPT-3, gbs=512 (~10^6 candidates)
 - 1xB200, HBM-roofline capture"), i.e. c3_homo64_mpl6 = 771 750 inter-stage plans, the configuration the
@@ -28,6 +28,14 @@ Timed regions
           of the same plans, one process per usable host core: the unmodified reference from baseline/_ref when
           that directory exists (kind "reference"), else the oracle (Python port of the pure-Python reference,
           oracle/metis_oracle.py, kind "port").
+
+--steps K sets the number of timed steps of every timed region: `value` and `e2e` of the headline workload and of
+each workload under `extra` (so a default run makes K end-to-end calls of the 68 M-plan configs[3] space too).
+
+--dump-outputs DIR writes, after the timed steps, what the last `value` search of the headline workload computed
+(the workloads under `extra` are not written): the costed candidates' records (records_cost, records_ordinal,
+records_step, records_num_repartition, records_num_stage, sorted by ordinal and step), counters and best, as float64
+.npy files.  The workloads are seeded, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -50,6 +58,7 @@ METRIC = 'candidate plans evaluated/sec'
 DEFAULT_WORKLOAD = 'c3_homo64_mpl6'
 EXTRA_WORKLOADS = ('c4_het128', 'c4_het128_mpl6')       # BASELINE configs[3] at max_permute_len 4 and 6
 REF_DIR = os.path.join(REPO, 'baseline', '_ref')
+DUMP_BYTES = 64_000_000                                   # --dump-outputs: at most this much in all
 
 
 def usable_cores():
@@ -288,8 +297,38 @@ class ClockSampler(threading.Thread):
                 'window': 'device-timed steps + end-to-end steps (both keep the GPU busy)'}
 
 
-def run_ours(ns, emit=True):
-    """One workload; rank 0 returns the JSON line (and prints it when ``emit``)."""
+def dump_outputs(out_dir, searcher):
+    """What the searcher's last search computed, as HetSearcher.run hands it to a caller: every costed candidate's
+    record in estimate_costs order (ordinal, then chain step), the counters and the best record, each as float64
+    (exact for these integers).  More than DUMP_BYTES of records are cut to a seeded sample of positions in that
+    order, whose indices are written too."""
+    from metis_b200 import native
+    sm = searcher.summary()
+    n = int(sm.num_records)
+    rec = searcher.records[:2 * n].cpu().numpy().view(native.RECORD_DTYPE)
+    rec = rec[np.lexsort((rec['step'], rec['ordinal']))]
+    fields = ('cost', 'ordinal', 'step', 'num_repartition', 'num_stage')
+    keep = (DUMP_BYTES - 4096) // (8 * (len(fields) + 1))    # 4 KiB for the small arrays and the .npy headers
+    out = {}
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        rec = rec[idx]
+        out['records_index'] = idx.astype(np.float64)
+    for f in fields:
+        out[f'records_{f}'] = rec[f].astype(np.float64)
+    out['counters'] = np.array([sm.num_records, sm.num_partition_calls, sm.num_balancer_runs, sm.num_keyerror],
+                               dtype=np.float64)
+    b = sm.best
+    out['best'] = np.array([b.cost, b.ordinal, b.step, b.num_repartition, b.num_stage] if n else [np.nan] * 5,
+                           dtype=np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), arr)
+
+
+def run_ours(ns, emit=True, dump_dir=None):
+    """One workload; rank 0 returns the JSON line (and prints it when ``emit``); with ``dump_dir`` every rank writes
+    the outputs of its last timed search there."""
     import torch
     import torch.distributed as dist
     from metis_b200 import api, flatten, native, search
@@ -402,9 +441,11 @@ def run_ours(ns, emit=True):
         dist.all_reduce(kmean, op=dist.ReduceOp.MAX)
     ms_per_step = float(total_ms.item()) / ns.steps
     kernel_ms = float(kmean.item())
+    if dump_dir:
+        dump_outputs(dump_dir if world == 1 else os.path.join(dump_dir, f'rank{rank}'), full)
 
     # ---- e2e: the drop-in API call from host inputs, every step -----------------------------------
-    e2e_steps = max(3, min(ns.steps, 10))
+    e2e_steps = ns.steps
     e2e_wall, parts = [], []
     res = None
     for i in range(e2e_steps + 2):                            # two warm-up calls: engine creation, buffer growth
@@ -518,7 +559,15 @@ def main():
     ap.add_argument('--cpu-sample', type=int, default=3000, help='plans per host core for cpu_baseline')
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--no-extra', action='store_true', help='skip the configs[3] measurements reported under `extra`')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed search computed as DIR/<name>.npy (float64): '
+                         'the headline workload only (not the workloads under `extra`); with --workload a,b '
+                         'DIR/<workload>/, with several ranks DIR/rank<r>/')
     ns = ap.parse_args()
+    if ns.steps < 1:
+        ap.error('--steps must be at least 1')
+    if ns.dump_outputs and ns.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU search (--impl ours)')
     # stdout carries exactly one JSON line: libraries that write to fd 1 (NCCL prints its version there when
     # NCCL_DEBUG=VERSION) are sent to stderr for the duration of the run
     global _RESULT_FD
@@ -532,13 +581,13 @@ def main():
     # this process group and prints one line each; the default invocation prints exactly one line
     names = ns.workload.split(',')
     if names == [DEFAULT_WORKLOAD] and not ns.no_extra:
-        # the headline line (BASELINE configs[2]) + the two configs[3] spaces, measured the same way with fewer steps,
-        # under `extra` (the 1 -> 8 scaling of the large spaces is where the GPUs pay off)
-        line = run_ours(ns, emit=False)
+        # the headline line (BASELINE configs[2]) + the two configs[3] spaces, measured the same way, under `extra`
+        # (the 1 -> 8 scaling of the large spaces is where the GPUs pay off)
+        line = run_ours(ns, emit=False, dump_dir=ns.dump_outputs)
         extra = {}
         for name in EXTRA_WORKLOADS:
             sub = argparse.Namespace(**vars(ns))
-            sub.workload, sub.steps, sub.no_cpu = name, min(ns.steps, 5), True
+            sub.workload, sub.no_cpu = name, True
             try:
                 other = run_ours(sub, emit=False)
             except Exception as exc:                          # noqa: BLE001 - the headline line must still be printed
@@ -555,7 +604,10 @@ def main():
     else:
         for name in names:
             ns.workload = name
-            run_ours(ns)
+            dump = ns.dump_outputs
+            if dump and len(names) > 1:
+                dump = os.path.join(dump, name)
+            run_ours(ns, dump_dir=dump)
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized():
         dist.destroy_process_group()

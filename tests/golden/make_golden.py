@@ -42,6 +42,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 REPO = os.path.dirname(os.path.dirname(HERE))
 REF = '/root/reference'
 sys.path.insert(0, REPO)
+sys.path.insert(0, os.path.dirname(HERE))           # tests/: golden_units, conftest
 
 from metis_b200.workloads import WORKLOADS, Workload, materialize, profile_file_order  # noqa: E402
 
@@ -237,10 +238,30 @@ def pack(rows):
     return out
 
 
+MAX_BYTES = 1_000_000
+CANDIDATE_KEYS = ('ordinal', 'step', 'ns_idx', 'batches', 'nrep', 'cost', 'label_stage', 'nstage', 'dp', 'tp', 'part')
+
+
 def save(name, meta, arrays):
+    """Writes tests/golden/<name>.npz without 'groups' (dp * tp; conftest.load_golden rebuilds it).  When the file
+    would exceed MAX_BYTES it keeps a seeded sample of the candidates, their positions in 'rows', and records the
+    whole list's digest and best in meta (read by conftest.assert_candidates_equal / golden_best)."""
+    from conftest import candidates_digest, golden_best
     path = os.path.join(HERE, f'{name}.npz')
+    arrays = {k: v for k, v in arrays.items() if k != 'groups'}
     np.savez_compressed(path, meta=np.array(json.dumps(meta)), **arrays)
-    print(f'wrote {path} ({os.path.getsize(path)} bytes)', file=sys.stderr)
+    n = len(arrays['cost'])
+    keep = n
+    while os.path.getsize(path) > MAX_BYTES:
+        if keep == n:
+            meta = dict(meta, best=list(golden_best({}, arrays)),
+                        digest=candidates_digest(arrays['ordinal'], arrays['step'], arrays['nrep'], arrays['nstage'],
+                                                 arrays['cost'], arrays['dp'], arrays['tp'], arrays['part']))
+        keep = int(keep * 0.95 * MAX_BYTES / os.path.getsize(path))
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        sub = {k: (v[rows] if k in CANDIDATE_KEYS else v) for k, v in arrays.items()}
+        np.savez_compressed(path, meta=np.array(json.dumps(meta)), rows=rows, **sub)
+    print(f'wrote {path} ({os.path.getsize(path)} bytes, {keep} of {n} candidates)', file=sys.stderr)
 
 
 def stratified_sample(w: Workload, fraction: float, seed: int = 4321):
@@ -412,7 +433,6 @@ def golden_units():
     """Unit-level vectors from reference functions on seeded random inputs."""
     ref = import_reference()
     from search_space.device_group import gen_dgroups_for_stages_with_variance, gen_device_group_shapes
-    rng = random.Random(7)
     # device-group rows: full tables for small cases
     dg = []
     for ndev in (4, 8, 16, 32):
@@ -422,47 +442,23 @@ def golden_units():
                     rows = gen_dgroups_for_stages_with_variance(stages, ndev, gen_device_group_shapes(ndev),
                                                                 variance, mpl)
                     dg.append({'ndev': ndev, 'variance': variance, 'mpl': mpl, 'stages': stages, 'rows': rows})
-    # LayerComputeBalancer.run
+    # LayerComputeBalancer.run and _adj_compute_performance on the seeded inputs of tests/golden_units.py; only the
+    # outputs are stored
+    from golden_units import unit_inputs
+    bal_in, adj_in = unit_inputs()
     LCB = ref['load_balancer'].LayerComputeBalancer
-    bal = []
-    for _ in range(3000):
-        L = rng.choice([6, 10, 12, 24, 33, 48, 80, 96])
-        S = rng.randint(1, min(L, 40))
-        lc = [0.02 + rng.random() * 0.05] + [1 + rng.random() * rng.choice([0.01, 0.3, 3.0]) for _ in range(L - 2)] + [0.03]
-        tot = sum(lc)
-        lc = [x / tot for x in lc]
-        mode = rng.random()
-        if mode < 0.4:
-            capa = [rng.random() + 0.05 for _ in range(S)]
-        elif mode < 0.7:
-            capa = [rng.choice([1.0, 2.0, 4.0]) for _ in range(S)]
-        else:
-            capa = [1.0 + 0.02 * rng.random() for _ in range(S)]
-        tc = sum(capa)
-        capa = [c / tc for c in capa]
-        if rng.random() < 0.15:
-            capa = [c * rng.uniform(0.5, 1.5) for c in capa]       # un-normalised (after re-weighting)
-        part, _ = LCB(S, L, list(capa), lc).run()
-        bal.append({'L': L, 'S': S, 'lc': [x.hex() for x in lc], 'capa': [c.hex() for c in capa], 'part': part})
-    # _adj_compute_performance
+    bal = [LCB(S, L, list(capa), lc).run()[0] for S, L, capa, lc in bal_in]
     llb_cls = ref['load_balancer'].LayerLoadBalancer
-    adj = []
     dummy = llb_cls.__new__(llb_cls)
+    adj = []
     with contextlib.redirect_stdout(io.StringIO()):
-        for _ in range(1500):
-            S = rng.randint(1, 24)
-            c = [rng.random() + 0.01 for _ in range(S)]
-            t = sum(c)
-            c = [x / t for x in c]
-            mc = [rng.choice([16384, 81920, 163840, 655360]) for _ in range(S)]
-            md = [0.001 + 5.0 * rng.random() * rng.choice([2e4, 1e5, 4e5]) for _ in range(S)]
+        for c, mc, md in adj_in:
             out = dummy._adj_compute_performance(list(c), list(mc), list(md))
-            adj.append({'c': [x.hex() for x in c], 'mc': mc, 'md': [x.hex() for x in md],
-                        'out': None if out is None else [x.hex() for x in out]})
+            adj.append(None if out is None else [x.hex() for x in out])
     path = os.path.join(HERE, 'units.json')
     import gzip
-    with gzip.open(path + '.gz', 'wt') as fh:
-        json.dump({'device_groups': dg, 'balancer': bal, 'adjust': adj}, fh)
+    with gzip.GzipFile(path + '.gz', 'wb', mtime=0) as fh:
+        fh.write(json.dumps({'device_groups': dg, 'balancer_part': bal, 'adjust_out': adj}).encode())
     print(f'wrote {path}.gz', file=sys.stderr)
 
 

@@ -11,7 +11,8 @@ import numpy as np
 import pytest
 
 import hostsim_util as hs
-from conftest import C1_DIR, GOLDEN, golden_rows, load_golden
+from conftest import C1_DIR, GOLDEN, assert_candidates_equal, device_columns, golden_rows, load_golden
+from golden_units import load_units
 from metis_b200 import flatten, native
 
 
@@ -105,8 +106,7 @@ def test_fatal_indexerror_unequal_nodes(name, mode, workload_dir):
 
 @pytest.fixture(scope='module')
 def units():
-    with gzip.open(os.path.join(GOLDEN, 'units.json.gz'), 'rt') as fh:
-        return json.load(fh)
+    return load_units()
 
 
 def test_units_enumerator(units):
@@ -171,15 +171,7 @@ def test_full_size_spaces_on_host(name, workload_dir):
     else:
         c = meta['counters']
         assert (summary.num_partition_calls, summary.num_balancer_runs, summary.num_records) == (c['B'], c['runs'], c['C'])
-    assert len(rec) == len(arr['cost'])
-    assert (rec['ordinal'].astype(np.int64) == arr['ordinal']).all() and (rec['step'] == arr['step']).all()
-    assert (rec['cost'].view(np.uint64) == arr['cost'].view(np.uint64)).all()
-    assert (rec['num_repartition'] == arr['nrep']).all()
-    S = arr['nstage'].astype(np.int64)
-    for i in range(0, len(rec), max(1, len(rec) // 2000)):          # partitions of a spread of candidates
-        s = int(S[i])
-        assert det[i, 2 * s:3 * s + 1].tolist() == arr['part'][i, :s + 1].tolist()
-        assert (1 << det[i, :s].astype(np.int64)).tolist() == arr['dp'][i, :s].tolist()
+    assert_candidates_equal(device_columns(rec, det, arr['dp'].shape[1]), meta, arr)
 
 
 @pytest.mark.parametrize('name,root_kind', [('c1', 'c1'), ('c3_homo64_mpl4', 'syn'), ('sweep_n8_t1', 'syn')])

@@ -13,7 +13,8 @@ import random
 import numpy as np
 import pytest
 
-from conftest import C1_DIR, GOLDEN, golden_rows, load_golden
+from conftest import C1_DIR, GOLDEN, assert_candidates_equal, device_columns, golden_best, golden_rows, load_golden
+from golden_units import load_units
 
 pytestmark = pytest.mark.gpu
 
@@ -55,31 +56,9 @@ def _cfg(w):
                 variance=w.variance, mpl=w.max_permute_len, max_tp=w.max_tp, max_bs=w.max_bs)
 
 
-def _assert_arrays_equal(out, space, arr):
-    """Vectorised comparison of sorted device records with the golden arrays."""
-    rec, det = out.records, out.detail
-    n = len(arr['cost'])
-    assert len(rec) == n
-    assert (rec['ordinal'].astype(np.int64) == arr['ordinal']).all()
-    assert (rec['step'].astype(np.int64) == arr['step']).all()
-    assert (rec['num_repartition'].astype(np.int64) == arr['nrep']).all()
-    assert (rec['num_stage'].astype(np.int64) == arr['nstage']).all()
-    assert (rec['cost'].view(np.uint64) == arr['cost'].view(np.uint64)).all(), 'fp64 cost bits differ'
-    smax = arr['dp'].shape[1]
-    S = arr['nstage'].astype(np.int64)
-    col = np.arange(smax)[None, :]
-    live = col < S[:, None]
-    rows = np.arange(n)[:, None]
-    wmax = det.shape[1] - 1
-    dp = 1 << det[rows, np.minimum(col, wmax)].astype(np.int64)
-    tp = 1 << det[rows, np.minimum(S[:, None] + col, wmax)].astype(np.int64)
-    assert (np.where(live, dp, 0) == np.where(live, arr['dp'], 0)).all()
-    assert (np.where(live, tp, 0) == np.where(live, arr['tp'], 0)).all()
-    colp = np.arange(smax + 1)[None, :]
-    livep = colp <= S[:, None]
-    part = det[rows, np.minimum(2 * S[:, None] + colp, wmax)].astype(np.int64)
-    assert (np.where(livep, part, 0) == np.where(livep, arr['part'], 0)).all()
-    assert (np.where(live, dp * tp, 0) == np.where(live, arr['groups'], 0)).all()
+def _assert_arrays_equal(out, space, arr, meta):
+    """Vectorised comparison of sorted device records with the golden (conftest.assert_candidates_equal)."""
+    assert_candidates_equal(device_columns(out.records, out.detail, arr['dp'].shape[1]), meta, arr)
 
 
 def test_c1_het_and_homo_vs_golden_and_oracle():
@@ -91,7 +70,7 @@ def test_c1_het_and_homo_vs_golden_and_oracle():
     problem, space, out = _device_search(meta, C1_DIR, 'profile_data_samples', w)
     assert space.num_plans == 32 and out.summary['num_records'] == 19
     assert out.summary['num_partition_calls'] == meta['counters']['B']
-    _assert_arrays_equal(out, space, arr)
+    _assert_arrays_equal(out, space, arr, meta)
     assert out.best[:3] == (621.8881853975784, 7, 0)
     # same inputs through the oracle (not the golden file)
     ocl = orc.OracleCluster(os.path.join(C1_DIR, 'hostfile'), os.path.join(C1_DIR, 'clusterfile.json'))
@@ -126,7 +105,7 @@ def test_synthetic_vs_golden(name, workload_dir):
     assert (s['num_partition_calls'], s['num_balancer_runs'], s['num_records'], s['num_keyerror']) == \
         (c['B'], c['runs'], c['C'], c['keyerr'])
     assert s['fatal_ordinal'] == 2 ** 64 - 1
-    _assert_arrays_equal(out, space, arr)
+    _assert_arrays_equal(out, space, arr, meta)
     gold = golden_rows(arr)
     best = min(gold, key=lambda g: (g[8], g[0], g[1]))
     assert out.best[:3] == (best[8], best[0], best[1])
@@ -144,9 +123,8 @@ def test_full_size_c3_vs_golden(name, workload_dir):
     assert space.num_plans == c['A']
     s = out.summary
     assert (s['num_partition_calls'], s['num_balancer_runs'], s['num_records']) == (c['B'], c['runs'], c['C'])
-    _assert_arrays_equal(out, space, arr)
-    i = int(np.lexsort((arr['step'], arr['ordinal'], arr['cost']))[0])
-    assert out.best[:3] == (float(arr['cost'][i]), int(arr['ordinal'][i]), int(arr['step'][i]))
+    _assert_arrays_equal(out, space, arr, meta)
+    assert out.best[:3] == golden_best(meta, arr)
 
 
 @pytest.mark.parametrize('env', [{'METIS_CHAIN_THREADS': '64'}, {'METIS_SMEM_BLOB_MAX': '0'},
@@ -165,7 +143,7 @@ def test_launch_shapes_give_the_same_records(env, workload_dir, monkeypatch):
     c = meta['counters']
     s = out.summary
     assert (s['num_partition_calls'], s['num_balancer_runs'], s['num_records']) == (c['B'], c['runs'], c['C'])
-    _assert_arrays_equal(out, space, arr)
+    _assert_arrays_equal(out, space, arr, meta)
 
 
 @pytest.mark.parametrize('name', ['c4_het128', 'c4_het128_mpl6', 'sweep_n128_t1_v0', 'sweep_n256_t2_v0'])
@@ -193,13 +171,13 @@ def test_sampled_vs_golden(name, workload_dir):
     rec = out.records
     keep = np.isin(rec['ordinal'].astype(np.int64), arr['sample'])
     sub = rec[keep]
-    assert len(sub) == len(arr['cost']) == meta['counters']['C']
+    assert len(sub) == meta['counters']['C']
     stride = 3 * int(space.blocks['num_stage'].max()) + 1
 
     class Sub:
         records = sub
         detail = searcher.detail_for(sub)[:, :max(stride, arr['dp'].shape[1] * 3 + 1)]
-    _assert_arrays_equal(Sub, space, arr)
+    _assert_arrays_equal(Sub, space, arr, meta)
     # every block of the space has sampled plans, and the blocks with costed candidates appear in the comparison
     blk_of = np.searchsorted(space.blocks['first_ordinal'], arr['sample'], side='right') - 1
     assert len(np.unique(blk_of)) == len(space.blocks)
@@ -302,8 +280,7 @@ def test_rerun_is_idempotent(workload_dir):
 def test_layer_balancer_units_on_gpu():
     _gpu()
     from metis_b200 import search
-    with gzip.open(os.path.join(GOLDEN, 'units.json.gz'), 'rt') as fh:
-        units = json.load(fh)
+    units = load_units()
     by_l = {}
     for case in units['balancer']:
         by_l.setdefault((case['L'], tuple(case['lc'])), []).append(case)
@@ -451,7 +428,7 @@ def test_scheduler_modes_agree(name, factor, workload_dir):
     c = meta['counters']
     assert (out.summary['num_partition_calls'], out.summary['num_balancer_runs'], out.summary['num_records']) == \
         (c['B'], c['runs'], c['C'])
-    _assert_arrays_equal(out, space, arr)
+    _assert_arrays_equal(out, space, arr, meta)
 
 
 def _api_inputs(name, workload_dir):

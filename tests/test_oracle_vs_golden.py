@@ -4,14 +4,13 @@ The golden files were produced by tests/golden/make_golden.py, which imports
 /root/reference in the build container.  Everything here is exact: candidate
 order, partitions, strategies and the bits of every fp64 cost.
 """
-import gzip
-import json
 import os
 import random
 
 import pytest
 
-from conftest import C1_DIR, GOLDEN, golden_rows, load_golden
+from conftest import C1_DIR, golden_rows, load_golden
+from golden_units import load_units
 from oracle import metis_oracle as orc
 
 
@@ -112,8 +111,7 @@ def test_fatal_indexerror_unequal_nodes(name, workload_dir):
 
 @pytest.fixture(scope='module')
 def units():
-    with gzip.open(os.path.join(GOLDEN, 'units.json.gz'), 'rt') as fh:
-        return json.load(fh)
+    return load_units()
 
 
 def test_units_device_groups(units):
