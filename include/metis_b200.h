@@ -257,6 +257,19 @@ int metis_sort_records(MetisRecord *records, int64_t n, int32_t mode, uint32_t *
                        int64_t workspace_bytes, void *stream);
 
 /*
+ * The min(k, n) first records of the METIS_SORT_RANKED order, without ordering all n (most-significant-digit radix
+ * select over the (cost, ordinal, step) key, then metis_sort_records on the selected records only).  Records with
+ * equal keys keep their input order, as in the sort.  k == 0 or n == 0 writes nothing.
+ *   records   [device] n records in any order (read only)
+ *   out       [device] min(k, n) records, ranked
+ *   idx_out   [device] optional min(k, n) uint32: idx_out[i] = input position of out[i]
+ *   workspace [device] metis_select_workspace_bytes(n, k) bytes
+ */
+int64_t metis_select_workspace_bytes(int64_t n, int64_t k);
+int metis_select_records(const MetisRecord *records, int64_t n, int64_t k, MetisRecord *out, uint32_t *idx_out,
+                         void *workspace, int64_t workspace_bytes, void *stream);
+
+/*
  * Host-side enumeration of gen_dgroups_for_stages_with_variance (search_space/device_group.py:93-107)
  * in reference order.  Writes log2 codes, num_stages bytes per row, into out (host memory) and
  * returns the number of rows, or METIS_E_CAPACITY if capacity_rows is too small (call with

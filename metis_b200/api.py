@@ -14,11 +14,13 @@ holders of inputs - every evaluation happens on the GPU (metis_b200.search).
   search_space/plan.py UniformPlanGenerator             UniformPlanGenerator  (host iterator)
   search_space/plan.py InterStagePlanGenerator          InterStagePlanGenerator (iterator over the plan space)
   cost_het_cluster.py cost_het_cluster()                cost_het_cluster()    -> GPU
+  cost_het_cluster(...) then sorted(...)[:k]            best_het_plans(..., k) -> GPU (no whole list)
   cost_homo_cluster.py cost_homo_cluster()              cost_homo_cluster()   -> GPU
 """
 from __future__ import annotations
 
 import argparse
+import operator
 import time
 from dataclasses import dataclass
 from itertools import permutations
@@ -160,23 +162,16 @@ class InterStagePlanGenerator:
                                  gbs=self.gbs)
 
 
-class HetSearchResult(Sequence):
-    """What cost_het_cluster() returns: the reference's list of 7-tuples
-    ``(node_sequence, device_groups, strategies, batches, layer_partition, num_repartition, cost)`` in
-    ``estimate_costs`` order (cost_het_cluster.py:44-46), as a read-only sequence whose tuples are built when they
-    are asked for (the columns live in numpy arrays; strategies / partitions stay on the GPU until needed).
-    ``len()``, indexing, slicing, iteration, ``sorted(result, key=...)`` and comparison with a list behave like the
-    reference's list.  ``ranked()`` is ``sorted(result, key=lambda kv: kv[6])`` (cost_het_cluster.py:76, a stable
-    sort) taken from the device sort's permutation instead of sorting Python objects."""
+class _TupleSequence(Sequence):
+    """A read-only sequence of the reference's 7-tuples
+    ``(node_sequence, device_groups, strategies, batches, layer_partition, num_repartition, cost)`` whose tuples are
+    built from ``candidates`` (search.Candidates) when they are asked for.  ``len()``, indexing, slicing, iteration,
+    ``sorted(result, key=...)`` and comparison with a list behave like a list's."""
 
-    def __init__(self, candidates, rank_order: Optional[np.ndarray], summary: Dict[str, int],
-                 timings: Optional[Dict[str, float]] = None, ranker=None, best_key: Optional[Tuple[int, int]] = None):
+    def __init__(self, candidates, summary: Dict[str, int], timings: Optional[Dict[str, float]] = None):
         self.candidates = candidates
-        self.rank_order = rank_order          # permutation of sorted(..., key=cost); computed on first use (``ranker``)
         self.summary = summary
         self.timings = timings or {}
-        self._ranker = ranker                 # () -> uint32 permutation, the stable device sort by cost
-        self._best_key = best_key             # (ordinal, step) of the argmin found by the search kernels
 
     def __len__(self) -> int:
         return len(self.candidates)
@@ -206,11 +201,30 @@ class HetSearchResult(Sequence):
 
     @property
     def costs(self) -> np.ndarray:
-        """fp64 cost of every candidate, estimate_costs order (no tuples built)."""
+        """fp64 cost of every entry, in the sequence's order (no tuples built)."""
         return self.candidates.cost
 
+
+class HetSearchResult(_TupleSequence):
+    """What cost_het_cluster() returns: the reference's list of 7-tuples in ``estimate_costs`` order
+    (cost_het_cluster.py:44-46), as a lazy read-only sequence (the columns live in numpy arrays; strategies /
+    partitions stay on the GPU until needed).  ``ranked()`` is ``sorted(result, key=lambda kv: kv[6])``
+    (cost_het_cluster.py:76, a stable sort) taken from the device sort's permutation instead of sorting Python
+    objects."""
+
+    def __init__(self, candidates, rank_order: Optional[np.ndarray], summary: Dict[str, int],
+                 timings: Optional[Dict[str, float]] = None, ranker=None, best_key: Optional[Tuple[int, int]] = None):
+        super().__init__(candidates, summary, timings)
+        self.rank_order = rank_order          # permutation of sorted(..., key=cost); computed on first use (``ranker``)
+        self._ranker = ranker                 # (k=None) -> uint32 permutation (or its first k), from the device
+        self._best_key = best_key             # (ordinal, step) of the argmin found by the search kernels
+
     def ranked(self, k: Optional[int] = None) -> List[Tuple]:
-        """The first ``k`` (default: all) entries of ``sorted(result, key=lambda kv: kv[6])``."""
+        """The first ``k`` (default: all) entries of ``sorted(result, key=lambda kv: kv[6])``.  Before the whole
+        ranking has been asked for, a ``k`` below ``len(self)`` is served by the device selection (only k records
+        are ordered)."""
+        if self.rank_order is None and self._ranker is not None and k is not None and 0 <= k < len(self):
+            return self.candidates.tuples(self._ranker(k))
         if self.rank_order is None:
             self.rank_order = self._ranker() if self._ranker is not None \
                 else np.argsort(self.candidates.cost, kind='stable')
@@ -288,6 +302,28 @@ def release_engines() -> None:
     _ENGINES.clear()
 
 
+def _prepare(args, gpu_cluster, profile_data, model_config, layer_load_balancer, node_sequences, device, corrected):
+    """What cost_het_cluster() and best_het_plans() share before the search: the corrections are checked, the inputs
+    flattened and staged on the device in the cached engine.  Returns (torch.distributed or None, problem, space,
+    node sequences, DeviceProblem, HetSearcher, perf_counter() when the flattening ended)."""
+    unknown = set(corrected) - {'Q1', 'Q2', 'Q5', 'Q6'}
+    if unknown:
+        raise ValueError(f'unknown corrections {sorted(unknown)}: choose from Q1, Q2, Q5, Q6')
+    import torch
+    from . import search
+    dist = torch.distributed if (torch.distributed.is_available() and torch.distributed.is_initialized()) else None
+    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
+    dev = search._require_cuda(device)
+    # the host lists the compositions (a few thousand records); the rows themselves are written by the GPU
+    problem, space, seqs = het_problem(args, gpu_cluster, profile_data, model_config, layer_load_balancer,
+                                       node_sequences, corrected=tuple(corrected), device_rows=True)
+    t1 = time.perf_counter()
+    stride = 3 * int(space.blocks['num_stage'].max()) + 1
+    dp, searcher = _engine(problem, space, dev, rank, world, stride)
+    dp.upload()
+    return dist, problem, space, seqs, dp, searcher, t1
+
+
 def cost_het_cluster(args: argparse.Namespace, gpu_cluster, profile_data: Dict, model_config: ModelConfig,
                      cost_estimator: HeteroCostEstimator, layer_load_balancer: LayerLoadBalancer,
                      node_sequences: Optional[Sequence[Sequence]] = None, device=None,
@@ -304,22 +340,10 @@ def cost_het_cluster(args: argparse.Namespace, gpu_cluster, profile_data: Dict, 
     takes a stage's memory demand from the profile of its own device type (load_balancer.py:41-52 uses the first
     type of the node sequence and, for mixed stages, sums a whole-cluster split).  Results of a corrected search are
     NOT the reference's; ``result.summary['corrected']`` records what was applied."""
-    unknown = set(corrected) - {'Q1', 'Q2', 'Q5', 'Q6'}
-    if unknown:
-        raise ValueError(f'unknown corrections {sorted(unknown)}: choose from Q1, Q2, Q5, Q6')
-    import torch
     from . import search
     t0 = time.perf_counter()
-    dist = torch.distributed if (torch.distributed.is_available() and torch.distributed.is_initialized()) else None
-    rank, world = (dist.get_rank(), dist.get_world_size()) if dist else (0, 1)
-    dev = search._require_cuda(device)
-    # the host lists the compositions (a few thousand records); the rows themselves are written by the GPU
-    problem, space, seqs = het_problem(args, gpu_cluster, profile_data, model_config, layer_load_balancer,
-                                       node_sequences, corrected=tuple(corrected), device_rows=True)
-    t1 = time.perf_counter()
-    stride = 3 * int(space.blocks['num_stage'].max()) + 1
-    dp, searcher = _engine(problem, space, dev, rank, world, stride)
-    dp.upload()
+    dist, problem, space, seqs, dp, searcher, t1 = _prepare(args, gpu_cluster, profile_data, model_config,
+                                                            layer_load_balancer, node_sequences, device, corrected)
     failure = None
     out = best = None
     try:
@@ -358,6 +382,68 @@ def cost_het_cluster(args: argparse.Namespace, gpu_cluster, profile_data: Dict, 
     result.timings = {'flatten_enumerate_s': t1 - t0, 'gpu_search_s': t2 - t1,
                       'decode_columns_s': time.perf_counter() - t2}
     return result
+
+
+# best_het_plans on one GPU: up to this many winners are replayed (metis_het_detail, one thread per winner walks its
+# whole strategy chain); more are gathered from detail rows the search writes.  On a B200 the replay of 1000 winners
+# cost 16 - 30 ms (profiles/r03_topk.md), more than the whole list's detail rows.
+_TOPK_REPLAY_MAX = 64
+
+
+class HetTopResult(_TupleSequence):
+    """What best_het_plans() returns: ``cost_het_cluster(...).ranked(k)`` - the k best 7-tuples in rank order - as a
+    lazy read-only sequence.  ``summary`` holds the counters of the WHOLE search (``num_records`` = C, not k)."""
+
+
+def best_het_plans(args: argparse.Namespace, gpu_cluster, profile_data: Dict, model_config: ModelConfig,
+                   cost_estimator: HeteroCostEstimator, layer_load_balancer: LayerLoadBalancer, k: int,
+                   node_sequences: Optional[Sequence[Sequence]] = None, device=None,
+                   corrected: Sequence[str] = ()) -> HetTopResult:
+    """The k best plans of cost_het_cluster() without producing the whole list: equal, tuple for tuple and bit for
+    bit, to ``cost_het_cluster(...).ranked(k)`` (lowest cost first, equal costs in estimate_costs order), and
+    raising what cost_het_cluster() raises.  The search writes no detail rows, the device selects the k best records
+    (metis_select_records), only those k records reach the host and their strategies and partitions are replayed.
+    With torch.distributed initialised every rank sends its k best to every other rank (instead of its whole list)
+    and every rank returns the same k."""
+    k = operator.index(k)
+    if k < 0:
+        raise ValueError(f'k must be >= 0, got {k}')
+    import torch
+    from . import search
+    t0 = time.perf_counter()
+    dist, problem, space, seqs, dp, searcher, t1 = _prepare(args, gpu_cluster, profile_data, model_config,
+                                                            layer_load_balancer, node_sequences, device, corrected)
+    failure = None
+    out = None
+    try:
+        # one GPU: few winners are replayed, many are gathered from detail rows written during the search
+        out = searcher.run_top(k, with_detail=dist is None and k > _TOPK_REPLAY_MAX)
+    except Exception as exc:                                  # noqa: BLE001 - re-raised below on every rank
+        if not dist:
+            raise
+        failure = exc
+    if dist:
+        def select(records, kk):
+            return searcher.select_records(records, records.numel() // 2, kk, torch.cuda.current_stream(dp.device))[0]
+        summary, _best, top = search.global_top(out.summary if out is not None else {},
+                                               out.best if out is not None else None,
+                                               out.records_dev if out is not None else None, k, dp.device, failure,
+                                               select)
+    else:
+        summary, top = out.summary, out.records_dev
+    if summary['fatal_ordinal'] != 2 ** 64 - 1:
+        search.raise_fatal(summary, problem)                  # quirk Q8, as in cost_het_cluster()
+    with torch.cuda.device(dp.device):
+        records = top.cpu().numpy().view(np.uint8).view(native.RECORD_DTYPE)
+        if out is not None and out.detail_dev is not None:
+            detail = out.detail_dev.cpu().numpy()
+        else:
+            detail = searcher.detail_for(records, stride=searcher.detail_stride) if len(records) else None
+    t2 = time.perf_counter()
+    cand = search.Candidates(records, detail, space, seqs, rows_dev=dp.rows_device().clone())
+    return HetTopResult(cand, dict(summary, num_plans=space.num_plans, corrected=tuple(sorted(corrected))),
+                        {'flatten_enumerate_s': t1 - t0, 'gpu_search_s': t2 - t1,
+                         'decode_columns_s': time.perf_counter() - t2})
 
 
 def cost_homo_cluster(args: argparse.Namespace, gpu_cluster, cost_estimator: HomoCostEstimator,

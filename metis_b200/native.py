@@ -80,7 +80,7 @@ COMP_DTYPE = [('row_offset', '<i8'), ('pool_offset', '<u4'), ('stages', '<u2'), 
 SYMBOLS = ['metis_last_error', 'metis_abi_version', 'metis_set_profile_events', 'metis_het_workspace_bytes', 'metis_het_search',
            'metis_het_detail', 'metis_het_trace', 'metis_homo_cost', 'metis_layer_balance', 'metis_enum_device_groups',
            'metis_enum_device_group_tables', 'metis_sort_workspace_bytes', 'metis_sort_records',
-           'metis_enum_compositions', 'metis_generate_rows']
+           'metis_enum_compositions', 'metis_generate_rows', 'metis_select_workspace_bytes', 'metis_select_records']
 SORT_POSITION, SORT_RANKED, SORT_BY_COST_STABLE = 0, 1, 2
 
 _lib = None
@@ -136,6 +136,11 @@ def load_library(path: str = LIB_PATH) -> C.CDLL:
     lib.metis_sort_workspace_bytes.argtypes = [C.c_int64]
     lib.metis_sort_records.restype = C.c_int
     lib.metis_sort_records.argtypes = [C.c_void_p, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.metis_select_workspace_bytes.restype = C.c_int64
+    lib.metis_select_workspace_bytes.argtypes = [C.c_int64, C.c_int64]
+    lib.metis_select_records.restype = C.c_int
+    lib.metis_select_records.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.c_int64, C.c_void_p]
     if lib.metis_abi_version() != 2:
         raise MetisNativeError('libmetis_b200.so ABI version mismatch; rebuild')
     if path == LIB_PATH:

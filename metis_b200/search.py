@@ -170,7 +170,7 @@ class HetSearcher:
                  want_ranking: bool = False, detail_to_host: bool = True, detail_stride: Optional[int] = None):
         self.dp = dp
         self.want_ranking = want_ranking and want_records
-        self._sort_ws = None
+        self._sort_ws = self._select_ws = None
         self.shard = native.MetisShard(rank, world, tile, 0)
         self.want_records = want_records
         self.want_detail = want_detail and want_records
@@ -205,14 +205,15 @@ class HetSearcher:
             self.detail = (torch.empty((capacity, self.detail_stride), dtype=torch.uint8, device=dev)
                            if self.want_detail else None)
 
-    def launch(self, stream: Optional[torch.cuda.Stream] = None) -> None:
+    def launch(self, stream: Optional[torch.cuda.Stream] = None, with_detail: bool = True) -> None:
         """Enqueue pack + search + finalize + summary copy on ``stream`` (asynchronous)."""
         dp = self.dp
         s = stream or torch.cuda.current_stream(dp.device)
+        detail = self.detail if with_detail else None
         rc = dp.lib.metis_het_search(
             C.byref(dp.p_struct), C.byref(dp.s_struct), C.byref(self.shard),
             C.c_void_p(self.records.data_ptr() if self.records is not None else 0), C.c_int64(self.capacity),
-            C.c_void_p(self.detail.data_ptr() if self.detail is not None else 0), C.c_int32(self.detail_stride),
+            C.c_void_p(detail.data_ptr() if detail is not None else 0), C.c_int32(self.detail_stride),
             C.c_void_p(self.workspace.data_ptr()), C.c_int64(self.workspace.numel()),
             C.c_void_p(self.summary_host.data_ptr()), C.c_void_p(s.cuda_stream))
         native.check(rc, 'metis_het_search')
@@ -246,29 +247,70 @@ class HetSearcher:
         slot[1] = weakref.ref(arr)
         return arr
 
+    def _search(self, s: torch.cuda.Stream, with_detail: bool = True):
+        """launch + synchronise; grows the record buffer and searches again when it was too small."""
+        self.launch(s, with_detail)
+        s.synchronize()
+        sm = self.summary()
+        if self.want_records and sm.num_records > self.capacity:
+            # C is not known before the first search of a space: size the buffers and search again
+            self._alloc(int(sm.num_records) + max(1024, int(sm.num_records) // 64))
+            self.launch(s, with_detail)
+            s.synchronize()
+            sm = self.summary()
+        out_summary = dict(num_records=int(sm.num_records), num_partition_calls=int(sm.num_partition_calls),
+                           num_balancer_runs=int(sm.num_balancer_runs), num_keyerror=int(sm.num_keyerror),
+                           fatal_ordinal=int(sm.fatal_ordinal), fatal_code=int(sm.fatal_code),
+                           fatal_aux=int(sm.fatal_aux), num_admitted=int(sm.reserved[0]),
+                           num_chained=int(sm.reserved[1]))
+        best = None
+        if sm.num_records > 0:
+            b = sm.best
+            best = (float(b.cost), int(b.ordinal), int(b.step), int(b.num_repartition), int(b.num_stage))
+        return sm, out_summary, best
+
+    def run_top(self, k: int, stream: Optional[torch.cuda.Stream] = None, with_detail: bool = False) -> HetSearchOutput:
+        """The search, then the shard's ``min(k, C)`` first records of the ranked order selected on the device
+        (``records_dev``, ranked, still on the device; ``records`` stays None).  Without detail rows the winners'
+        strategies and partitions come from ``detail_for`` afterwards; ``with_detail`` (a searcher that has detail
+        rows) writes them during the search and gathers the winners' rows into ``detail_dev``."""
+        dp = self.dp
+        s = stream or torch.cuda.current_stream(dp.device)
+        with_detail = with_detail and self.want_detail
+        with torch.cuda.device(dp.device):
+            _sm, out_summary, best = self._search(s, with_detail=with_detail)
+            n = out_summary['num_records']
+            top, idx = self.select_records(self.records, n, k, s, want_idx=with_detail)
+            detail_dev = self.detail[:n].index_select(0, idx.long()) if with_detail else None
+        return HetSearchOutput(out_summary, best, None, None, C.sizeof(native.MetisSearchSummary), records_dev=top,
+                               detail_dev=detail_dev)
+
+    def select_records(self, buf: torch.Tensor, n: int, k: int, stream: torch.cuda.Stream, want_idx: bool = False):
+        """metis_select_records on the first n records of ``buf`` (asynchronous on ``stream``): the ranked
+        ``min(k, n)`` first records as a new int64 tensor, and their positions in ``buf`` (int32 view of the uint32
+        indices) when asked."""
+        dp = self.dp
+        m = min(k, n)
+        need = int(dp.lib.metis_select_workspace_bytes(C.c_int64(n), C.c_int64(k)))
+        if need < 0:
+            native.check(need, 'metis_select_workspace_bytes')
+        if self._select_ws is None or self._select_ws.numel() < need:
+            self._select_ws = torch.empty(need + need // 8, dtype=torch.uint8, device=dp.device)
+        top = torch.empty(2 * max(m, 1), dtype=torch.int64, device=dp.device)
+        idx = torch.empty(max(m, 1), dtype=torch.int32, device=dp.device) if want_idx else None
+        rc = dp.lib.metis_select_records(C.c_void_p(buf.data_ptr()), C.c_int64(n), C.c_int64(k),
+                                         C.c_void_p(top.data_ptr()), C.c_void_p(idx.data_ptr() if idx is not None else 0),
+                                         C.c_void_p(self._select_ws.data_ptr()), C.c_int64(self._select_ws.numel()),
+                                         C.c_void_p(stream.cuda_stream))
+        native.check(rc, 'metis_select_records')
+        return top[:2 * m], (idx[:m] if idx is not None else None)
+
     def run(self, stream: Optional[torch.cuda.Stream] = None) -> HetSearchOutput:
         """launch + synchronise + bring results to the host; grows the record buffer if needed."""
         dp = self.dp
         s = stream or torch.cuda.current_stream(dp.device)
         with torch.cuda.device(dp.device):
-            self.launch(s)
-            s.synchronize()
-            sm = self.summary()
-            if self.want_records and sm.num_records > self.capacity:
-                # C is not known before the first search of a space: size the buffers and search again
-                self._alloc(int(sm.num_records) + max(1024, int(sm.num_records) // 64))
-                self.launch(s)
-                s.synchronize()
-                sm = self.summary()
-            out_summary = dict(num_records=int(sm.num_records), num_partition_calls=int(sm.num_partition_calls),
-                               num_balancer_runs=int(sm.num_balancer_runs), num_keyerror=int(sm.num_keyerror),
-                               fatal_ordinal=int(sm.fatal_ordinal), fatal_code=int(sm.fatal_code),
-                               fatal_aux=int(sm.fatal_aux), num_admitted=int(sm.reserved[0]),
-                               num_chained=int(sm.reserved[1]))
-            best = None
-            if sm.num_records > 0:
-                b = sm.best
-                best = (float(b.cost), int(b.ordinal), int(b.step), int(b.num_repartition), int(b.num_stage))
+            sm, out_summary, best = self._search(s)
             records = detail = rank_order = detail_dev = records_dev = None
             d2h = C.sizeof(native.MetisSearchSummary)
             if self.want_records:
@@ -307,16 +349,17 @@ class HetSearcher:
         native.check(rc, 'metis_sort_records')
         return perm[:n] if perm is not None else None
 
-    def detail_for(self, picks: np.ndarray, stream: Optional[torch.cuda.Stream] = None) -> np.ndarray:
-        """Strategies and partition of chosen records (metis_het_detail replay)."""
+    def detail_for(self, picks: np.ndarray, stream: Optional[torch.cuda.Stream] = None,
+                   stride: int = native.DETAIL_STRIDE) -> np.ndarray:
+        """Strategies and partition of chosen records (metis_het_detail replay), ``stride`` bytes per row."""
         dp = self.dp
         s = stream or torch.cuda.current_stream(dp.device)
         n = len(picks)
         with torch.cuda.device(dp.device):
             raw = torch.from_numpy(np.ascontiguousarray(picks).view(np.uint8).reshape(-1).copy()).to(dp.device)
-            out = torch.zeros((max(n, 1), native.DETAIL_STRIDE), dtype=torch.uint8, device=dp.device)
+            out = torch.zeros((max(n, 1), stride), dtype=torch.uint8, device=dp.device)
             rc = dp.lib.metis_het_detail(C.byref(dp.p_struct), C.byref(dp.s_struct), C.c_void_p(raw.data_ptr()),
-                                         C.c_int64(n), C.c_void_p(out.data_ptr()), C.c_int32(native.DETAIL_STRIDE),
+                                         C.c_int64(n), C.c_void_p(out.data_ptr()), C.c_int32(stride),
                                          C.c_void_p(self.workspace.data_ptr()), C.c_int64(self.workspace.numel()),
                                          C.c_void_p(s.cuda_stream))
             native.check(rc, 'metis_het_detail')
@@ -515,17 +558,49 @@ def global_exchange(summary: Dict[str, int], local_best, device, local_error: in
     return _merge_counters(summary, [r[:8] for r in rows]), _pick_best([r[8:] for r in rows])
 
 
+def global_top(summary: Dict[str, int], local_best, local_top: Optional[torch.Tensor], k: int, device,
+               failure: Optional[BaseException] = None, select=None):
+    """The multi-rank step of a top-k search.  The counters, the error flag and the fatal plan travel in the one
+    96-byte ``global_exchange``; a rank whose search raised (``failure``) makes every rank raise.  Without a fatal
+    plan each rank's ``min(k, C_r)`` ranked records (``local_top``: int64 [2 m] on ``device``) are all-gathered,
+    k slots per rank, and ``select(records, k)`` picks the global first k from the merged ones.  Returns
+    (summary, best, top records or None when a plan was fatal)."""
+    import torch.distributed as dist
+    merged, best = global_exchange(summary, local_best, device, int(failure is not None))
+    if merged['any_rank_failed']:
+        raise failure if failure is not None else native.MetisNativeError('the search failed on another rank')
+    if merged['global_fatal_ordinal'] < 2 ** 62:
+        merged.update(fatal_ordinal=merged['global_fatal_ordinal'], fatal_code=merged['global_fatal_code'],
+                      fatal_aux=merged['global_fatal_aux'])
+        return merged, best, None
+    merged['fatal_ordinal'] = 2 ** 64 - 1
+    world = dist.get_world_size()
+    counts = [min(k, c) for c in merged['records_per_rank']]
+    cap = max(max(counts), 1)
+    mine = counts[dist.get_rank()]
+    pad = torch.zeros(2 * cap, dtype=torch.int64, device=device)
+    pad[:2 * mine] = local_top[:2 * mine]
+    gathered = torch.empty(2 * cap * world, dtype=torch.int64, device=device)
+    dist.all_gather_into_tensor(gathered, pad)
+    every = torch.cat([gathered[2 * cap * r:2 * cap * r + 2 * counts[r]] for r in range(world)]).contiguous()
+    return merged, best, select(every, k)
+
+
 def make_ranker(searcher: 'HetSearcher', records_dev: torch.Tensor):
-    """() -> permutation of ``sorted(records, key=cost)`` (stable): the device sort on a private copy of the ordered
-    records, run when a caller first asks for the ranking."""
+    """(k=None) -> permutation of ``sorted(records, key=cost)`` (stable), or its first k entries: the device sort, or
+    for a k the device selection, on a private copy of the ordered records, run when a caller first asks."""
     snap = records_dev.clone()
     n = snap.numel() // 2
     dev = searcher.dp.device
 
-    def rank() -> np.ndarray:
+    def rank(k: Optional[int] = None) -> np.ndarray:
         with torch.cuda.device(dev):
             s = torch.cuda.current_stream(dev)
-            perm = searcher.sort_records(n, native.SORT_BY_COST_STABLE, s, want_perm=True, buf=snap)
+            if k is None:
+                perm = searcher.sort_records(n, native.SORT_BY_COST_STABLE, s, want_perm=True, buf=snap)
+            else:
+                # the records are in position order, so the selection's input positions index estimate_costs
+                _, perm = searcher.select_records(snap, n, k, s, want_idx=True)
             s.synchronize()
             return perm.cpu().numpy().view(np.uint32)
     return rank

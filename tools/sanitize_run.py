@@ -25,3 +25,13 @@ for name in sys.argv[1:] or ['c2_v100', 'mix32']:
         s.shard.reserved = coop
         out = s.run()
         print(name, 'coop factor', coop, out.summary['num_records'], out.best[:3], 'ranked first', int(out.rank_order[0]))
+    # top-k path: the local selection on the search's unordered records, then a merge selection over two lists
+    import torch
+    t = search.HetSearcher(dp, want_records=True, want_detail=False)
+    top = t.run_top(10)
+    both = torch.cat([top.records_dev, out.records_dev]).contiguous()
+    merged, idx = t.select_records(both, both.numel() // 2, 10, torch.cuda.current_stream(), want_idx=True)
+    picks = merged.cpu().numpy().view('u1').view(search.native.RECORD_DTYPE)
+    rows = t.detail_for(picks)
+    torch.cuda.synchronize()
+    print(name, 'top-k', top.records_dev.numel() // 2, 'merged first', picks[0], 'from', int(idx[0]), rows.shape)
